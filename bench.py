@@ -4,6 +4,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload kafka|flat|wide] [--records R]
     python bench.py --impl reference ...        # the CPU arm: the oracle port on the usable host cores
     python bench.py --gpus N --gather ...        # C5: shards decoded per GPU, then gathered into single RecordBatches
+    python bench.py --dump-outputs DIR ...       # also write the last timed step's output to DIR/*.npy (dump_outputs)
 
 A "step" is one pass of the hot path over one batch of synthetic Avro records (C3: 10 M records, 8 output chunks):
   value     records/s with the packed input already resident in HBM and the Arrow buffers left in HBM
@@ -56,7 +57,14 @@ def parse_args():
     ap.add_argument("--seed", type=int, default=42)
     ap.add_argument("--gather", action="store_true", help="C5: gather the shards' batches into single RecordBatches on rank 0")
     ap.add_argument("--no-extras", action="store_true", help="skip C1/C2/C4, encode and the CPU baseline (main line only)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed device-resident step's output (a seeded sample of "
+                    "its rows, every Arrow array flattened to float32/float64) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.gather):
+        ap.error("--dump-outputs applies to the GPU arm's main line (not --impl reference or --gather)")
+    return args
 
 
 def config_of(args, world):
@@ -261,9 +269,11 @@ class Bench:
             raise SystemExit("rv_decode_host: " + self.pr._last_error())
         return h
 
-    def time_device(self, w, k, steps, warmup, sampler=None):
-        """Device-resident decode: CUDA events around `steps` calls, max over ranks."""
+    def time_device(self, w, k, steps, warmup, sampler=None, keep_last=False):
+        """Device-resident decode: CUDA events around `steps` calls, max over ranks.  With keep_last the last step's
+        result handle is returned as "last" instead of freed (the caller frees it)."""
         torch, L = self.torch, self.L
+        last = None
         arrow_bytes = buffer_bytes = 0
         for _ in range(warmup):
             h = self.step_device(w, k)
@@ -278,14 +288,17 @@ class Bench:
             sampler.active.set()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(self.stream)
-        for _ in range(steps):
+        for i in range(steps):
             h = self.step_device(w, k)
             L.rv_last_timings(tbuf, 6)
             kt += np.frombuffer(tbuf, dtype=np.float32)
             launches += L.rv_last_launch_count()
             passes = max(passes, L.rv_last_passes())
             slow += L.rv_last_slow_tiles()
-            L.rv_result_free(h)
+            if keep_last and i == steps - 1:
+                last = h
+            else:
+                L.rv_result_free(h)
         e1.record(self.stream)
         torch.cuda.synchronize()
         if sampler:
@@ -293,7 +306,7 @@ class Bench:
         self.barrier()
         ms_total = self.max_over_ranks(e0.elapsed_time(e1))
         return {"ms_per_step": ms_total / steps, "kernel_ms": kt / steps, "launches": launches, "passes": passes, "slow_tiles": slow,
-                "arrow_bytes": arrow_bytes, "buffer_bytes": buffer_bytes}
+                "arrow_bytes": arrow_bytes, "buffer_bytes": buffer_bytes, "last": last}
 
     def time_host(self, w, k, steps, warmup, sampler=None):
         """End to end through rv_decode_host (pinned host in, pinned host out), wall clock, max over ranks."""
@@ -406,6 +419,95 @@ def parity_check(b, w, k):
     pr._check(L.rv_result_to_host(h))
     assert_matches_oracle(co, pr._export_batches(h.value, w["schema"]), w["schema_json"], w["h_data"], w["h_off"], w["n"], k, full_validate=False)
     return True
+
+
+DUMP_MAX_BYTES = 64 << 20
+DUMP_MAX_ROWS = 1 << 15
+
+
+def flatten_arrow(name, arr, out):
+    """One Arrow array -> numpy float arrays in `out`, keyed by dotted path: validity (1/0), list and map lengths, union
+    type ids, string and binary lengths and bytes, fixed-width values.  A 64-bit integer becomes a (high, low) pair of
+    32-bit halves so that float64 holds it exactly."""
+    import pyarrow as pa
+    import pyarrow.compute as pc
+    t, n = arr.type, len(arr)
+    if not pa.types.is_union(t):          # a union has no validity of its own: its children carry it
+        out[name + ".valid"] = arr.is_valid().to_numpy(zero_copy_only=False).astype(np.float32)
+    if pa.types.is_struct(t):
+        for i in range(t.num_fields):
+            flatten_arrow(name + "." + t.field(i).name, arr.field(i), out)
+    elif pa.types.is_list(t) or pa.types.is_large_list(t) or pa.types.is_map(t):
+        off = arr.offsets.to_numpy().astype(np.int64)
+        lens = np.diff(off)
+        lens[~arr.is_valid().to_numpy(zero_copy_only=False)] = 0    # what a null list spans is not part of the value
+        out[name + ".len"] = lens.astype(np.float32)
+        ends = np.cumsum(lens)
+        items = np.arange(int(ends[-1]) if n else 0) + np.repeat(off[:-1] - (ends - lens), lens)
+        flatten_arrow(name + ".item", arr.values.take(pa.array(items, type=pa.int64())), out)
+    elif pa.types.is_union(t):
+        out[name + ".type_id"] = arr.type_codes.to_numpy().astype(np.float32)
+        if t.mode == "dense":
+            out[name + ".offset"] = arr.offsets.to_numpy().astype(np.float64)
+        for i in range(t.num_fields):
+            flatten_arrow(name + "." + t.field(i).name, arr.field(i), out)
+    elif pa.types.is_dictionary(t):
+        flatten_arrow(name + ".index", arr.indices, out)
+        flatten_arrow(name + ".dictionary", arr.dictionary, out)
+    elif pa.types.is_null(t):
+        pass
+    elif pa.types.is_boolean(t):
+        out[name] = arr.fill_null(False).to_numpy(zero_copy_only=False).astype(np.float32)
+    elif pa.types.is_fixed_size_binary(t):
+        raw = np.frombuffer(arr.buffers()[1], dtype=np.uint8)
+        out[name + ".bytes"] = raw[arr.offset * t.byte_width:(arr.offset + n) * t.byte_width].astype(np.float32)
+    elif pa.types.is_binary(t) or pa.types.is_string(t) or pa.types.is_large_binary(t) or pa.types.is_large_string(t):
+        out[name + ".len"] = pc.binary_length(arr).fill_null(0).to_numpy().astype(np.float32)
+        odt = np.int64 if pa.types.is_large_binary(t) or pa.types.is_large_string(t) else np.int32
+        bufs = arr.buffers()
+        off = np.frombuffer(bufs[1], dtype=odt)[arr.offset:arr.offset + n + 1]
+        data = np.frombuffer(bufs[2], dtype=np.uint8) if bufs[2] is not None else np.zeros(0, dtype=np.uint8)
+        out[name + ".bytes"] = data[off[0]:off[-1]].astype(np.float32)
+    else:                                 # fixed width: integers, floats, temporal types, decimals
+        width = t.bit_width // 8
+        raw = np.frombuffer(arr.buffers()[1], dtype=np.uint8)[arr.offset * width:(arr.offset + n) * width]
+        if pa.types.is_floating(t):
+            v = raw.view({2: np.float16, 4: np.float32, 8: np.float64}[width])
+            out[name] = v.astype(np.float32 if width <= 4 else np.float64)
+        elif width in (1, 2, 4) and not pa.types.is_decimal(t):
+            out[name] = raw.view({1: np.int8, 2: np.int16, 4: np.int32}[width]).astype(np.float64)
+        elif width == 8:
+            v = raw.view(np.int64)
+            out[name] = np.stack([v >> 32, v & 0xFFFFFFFF], axis=-1).astype(np.float64)
+        else:
+            out[name + ".bytes"] = raw.astype(np.float32)
+
+
+def dump_outputs(b, w, h, directory, seed):
+    """The decoded batches of result handle `h` (freed here) -> DIR/<name>.npy: `_batch_rows` (rows per output batch),
+    `_sample_rows` (the rows dumped: all of them, or a sample drawn with `seed`, sorted) and every column of those rows
+    through flatten_arrow.  The sample halves until the files fit in DUMP_MAX_BYTES."""
+    import pyarrow as pa
+    pr = b.pr
+    pr._check(b.L.rv_result_to_host(h))
+    batches = pr._export_batches(h.value, w["schema"])
+    table = pa.Table.from_batches(batches)
+    n = table.num_rows
+    rows = min(n, DUMP_MAX_ROWS)
+    while True:
+        idx = np.sort(np.random.default_rng(seed).choice(n, rows, replace=False)) if rows < n else np.arange(n)
+        sub = table.take(pa.array(idx)).combine_chunks()
+        out = {"_batch_rows": np.array([x.num_rows for x in batches], dtype=np.float64), "_sample_rows": idx.astype(np.float64)}
+        for name, col in zip(sub.column_names, sub.columns):
+            flatten_arrow(name, col.chunk(0) if col.num_chunks == 1 else pa.concat_arrays(col.chunks), out)
+        total = sum(a.nbytes for a in out.values())
+        if total <= DUMP_MAX_BYTES or rows == 1:
+            break
+        rows //= 2
+    os.makedirs(directory, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+    return {"dir": directory, "rows": int(len(idx)), "of_rows": n, "arrays": len(out), "bytes": int(total)}
 
 
 def c1_line(b):
@@ -566,7 +668,7 @@ def main():
                "--master-addr", "127.0.0.1", "--master-port", port, os.path.abspath(__file__)] + sys.argv[1:]
         sys.exit(subprocess.call(cmd))
 
-    steps, warmup = max(1, args.steps), max(3, args.warmup)
+    steps, warmup = args.steps, max(3, args.warmup)
 
     if args.impl == "reference":
         if rank == 0:
@@ -600,7 +702,9 @@ def main():
     if sampler:
         sampler.start()
 
-    dev_res = b.time_device(w, k, steps, warmup, sampler)
+    dump = args.dump_outputs if rank == 0 else None   # rank 0's shard: the first `records` rows
+    dev_res = b.time_device(w, k, steps, warmup, sampler, keep_last=bool(dump))
+    dumped = dump_outputs(b, w, dev_res.pop("last"), dump, args.seed) if dump else None
     host_res = b.time_host(w, k, steps, warmup, sampler)
     if sampler:
         sampler.stop()
@@ -629,6 +733,8 @@ def main():
         "roofline": rl,
         "clocks": sampler.summary() if sampler else None,
     }
+    if dumped:
+        line["dumped_outputs"] = dumped
     if world > 1:
         line["rank_binding"] = {"rank0_numa_node": numa_node, "how": "each rank's threads run on the CPUs of its GPU's NUMA node (bench.py: bind_to_gpu_node)"}
     if world == 1 and not args.no_extras:

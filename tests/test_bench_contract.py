@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -37,6 +39,58 @@ def test_usable_cores_respects_affinity_and_quota():
     assert 1 <= n <= aff
     if quota is not None:
         assert n <= max(1, int(quota + 0.999))
+
+
+def test_steps_below_one_is_an_error():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"], capture_output=True,
+                         text=True, timeout=120, cwd=ROOT)
+    assert out.returncode != 0 and "--steps" in out.stderr
+
+
+@pytest.mark.parametrize("workload", ["kafka", "flat", "wide"])
+def test_dump_flattening_keeps_every_value(workload, coracle):
+    """`--dump-outputs` writes each column through bench.flatten_arrow: float32/float64 arrays from which the rows can be
+    read back exactly (here from batches the C oracle decodes, sliced so that the arrays carry offsets)."""
+    import numpy as np
+    import pyarrow as pa
+    sys.path.insert(0, ROOT)
+    import bench
+    import workloads
+    from oracle import pyoracle as po
+    n = 3000
+    sj, data, off = workloads.generate(workload, n, seed=5)
+    recs = [data[off[i]:off[i + 1]].tobytes() for i in range(n)]
+    batch = po.canon_to_batch(coracle.decode(sj, recs), po.to_arrow_schema(po.parse_schema(sj))).slice(1000, 1500)
+    out = {}
+    for name, col in zip(batch.schema.names, batch.columns):
+        bench.flatten_arrow(name, col, out)
+    assert all(a.dtype in (np.float32, np.float64) for a in out.values())
+    assert 0 < sum(a.nbytes for a in out.values()) < 64 * 1500 * 1024
+
+    def text(prefix, row):
+        lens = out[prefix + ".len"].astype(np.int64)
+        start = int(lens[:row].sum())
+        return bytes(out[prefix + ".bytes"][start:start + lens[row]].astype(np.uint8)).decode()
+
+    def i64(prefix, row):
+        hi, lo = out[prefix][row]
+        return int(hi) * 2 ** 32 + int(lo)
+
+    rows = batch.to_pylist()
+    for r in (0, 1, 777, 1499):
+        want = rows[r]
+        if workload == "flat":
+            assert (out["i"][r], i64("l", r), out["f"][r], out["d"][r], out["b"][r]) == (want["i"], want["l"], want["f"], want["d"], want["b"])
+            assert text("s", r) == want["s"]
+        elif workload == "kafka":
+            assert i64("created_at", r) == want["created_at"] and text("class", r) == want["class"]
+            assert out["name.valid"][r] == (want["name"] is not None) and (want["name"] is None or text("name", r) == want["name"])
+            assert out["emails.len"][r] == len(want["emails"]) and out["phone_numbers.len"][r] == len(want["phone_numbers"])
+        else:
+            assert i64("id", r) == want["id"] and out["ml.len"][r] == len(want["ml"])
+    if workload == "kafka":
+        assert len(out["emails.item.valid"]) == sum(len(x["emails"]) for x in rows)
+        assert len(out["phone_numbers.item.keys.len"]) == sum(len(x["phone_numbers"]) for x in rows)
 
 
 def test_roofline_traffic_comes_from_a_committed_capture():
